@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the denoising hot path (BASELINE.json metric: denoising-steps/sec).
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload NAME] [--no-secondary]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload NAME] [--no-secondary] [--dump-outputs DIR]
 
 One "step" = one DDIM step of the workload's whole per-GPU batch: Beff U-Net evaluations (2B with
 classifier-free guidance) + the CFG/DDIM update.  Default workload = BASELINE.json configs[1]:
@@ -323,8 +323,7 @@ def measure(model, name, wl, steps, warmup, world, rank, dev, with_roofline=True
             for _ in range(10):
                 step()
             torch.cuda.synchronize()
-    if budget[0] < steps:
-        restart()
+    restart()                                   # the timed steps start from x_T at step 0, whatever the sustain phase ran
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     torch.cuda.synchronize()
     if world > 1:
@@ -343,7 +342,10 @@ def measure(model, name, wl, steps, warmup, world, rank, dev, with_roofline=True
     clock_info = clocks.stop() if rank == 0 else None
     launches_per_step = sess.plan.launches + 2
     value = world * steps / (ms / 1000.0)
-    finite = bool(torch.isfinite(sess.read_rows(sess.eps, Beff, 16, L)).all())
+    # what the last timed step computed: the latent after its DDIM update and the U-Net output it used (read here: the
+    # roofline below reuses the session's buffers)
+    outputs = dict(x=sess.read_rows(sess.xin.r(0, B * L), B, 16, L).cpu(), eps=sess.read_rows(sess.eps, Beff, 16, L).cpu())
+    finite = bool(torch.isfinite(outputs["eps"]).all())
 
     # ---- roofline of the dominant kernel family (GEMM) -----------------------------------------------------
     # Device time per kernel family, measured live with CUDA events: the ops of one family are put in their own
@@ -438,12 +440,13 @@ def measure(model, name, wl, steps, warmup, world, rank, dev, with_roofline=True
         times.append(float(dt.item()))
     dt = torch.tensor([sorted(times)[1]], device=dev)
     n_steps_e2e = len(sampler.ddim_timesteps)
+    outputs["e2e_logits"] = out.clone()
     e2e = dict(value=world * n_steps_e2e / float(dt.item()), unit=UNIT, h2d_bytes_per_step=h2d / n_steps_e2e,
                d2h_bytes_per_step=out.numel() * 4 / n_steps_e2e, request_ms=1000.0 * float(dt.item()), request_ms_all=[round(1000.0 * t, 2) for t in times], steps_in_request=n_steps_e2e,
                note=f"median of 3 sampler.sample(S={S}) + decode requests per GPU from pinned host inputs to pinned host logits; "
                     f"{n_steps_e2e} DDIM steps; per-step bytes = request bytes / steps")
     return dict(value=value, ms_per_step=ms / steps, e2e=e2e, roofline=roof, launches_per_step=launches_per_step, clocks=clock_info,
-                finite=finite, sampler=sampler, host=host, Beff=Beff)
+                finite=finite, sampler=sampler, host=host, Beff=Beff, outputs=outputs)
 
 
 def main():
@@ -458,7 +461,14 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-secondary", action="store_true", help="skip the secondary workloads (configs 3/4/5)")
     ap.add_argument("--cpu-steps", type=int, default=10)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write rank 0's outputs of the headline workload as float32 DIR/<name>.npy: x (latent after the last timed "
+                         "step), eps (U-Net output of that step) and e2e_logits (decoder logits of the last end-to-end request)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to --impl b200")
     name = args.workload
     wl = WORKLOADS[name]
     if args.impl == "reference":
@@ -479,6 +489,10 @@ def main():
     model, sd = build_model(L, world, rank, dev, args.gemm)
     eng = model.engine
     m = measure(model, name, wl, args.steps, args.warmup, world, rank, dev)
+    if args.dump_outputs and rank == 0:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for k, v in m["outputs"].items():
+            np.save(os.path.join(args.dump_outputs, k + ".npy"), v.numpy())
 
     # ---- secondary numbers: the same loop without guidance, the decode, and the other BASELINE configs -----------------------
     secondary = None

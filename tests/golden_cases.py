@@ -104,3 +104,31 @@ PROMPT_DICTS = [
     {"sr": 4.19999, "rank_status": "graveyard", "ln": False, "stamina": True, "stream_ett": 17.9},
     {"sr": 7.999, "rank_status": "loved", "hb": 0, "ln_ratio": 0.95},
 ]
+
+# a spec that exercises what the shipped yaml does not: count > 1 and non-integer bin edges
+PROMPT_SPEC_COUNT = [
+    {"name": "a", "type": "numeric", "min": 0.5, "max": 2.0, "interval": 0.25, "count": 3},
+    {"name": "b", "type": "category", "category": ["x", "y"], "count": 2},
+    {"name": "c", "type": "bool"},
+    {"name": "d", "type": "numeric", "min": -3, "max": 3, "interval": 1},
+]
+
+
+def random_feature_dicts(spec, n, rnd):
+    """n feature dicts drawn from ``rnd`` (a random.Random): features left out, values below / above the range, at its
+    edges and inside it; the ids the reference gives them are in tests/golden/prompt_random.json"""
+    out = []
+    for _ in range(n):
+        d = {}
+        for x in spec:
+            if rnd.random() < 0.4:
+                continue
+            if x["type"] == "numeric":
+                span = x["max"] - x["min"]
+                d[x["name"]] = rnd.choice([x["min"] - 1, x["max"] + 1, x["min"] + span * rnd.random(), x["min"], x["max"]])
+            elif x["type"] == "bool":
+                d[x["name"]] = rnd.choice([True, False, 0, 1])
+            else:
+                d[x["name"]] = rnd.choice(x["category"])
+        out.append(d)
+    return out

@@ -1,7 +1,6 @@
 """mug_diffusion_b200/postprocess.py (SURVEY §8f N4: gridify + mini-jack removal) against golden vectors produced by the UNMODIFIED
-reference (tools/make_postprocess_goldens.py -> tests/golden/postprocess.json), and against the live reference where its tree exists.
+reference (tools/make_postprocess_goldens.py -> tests/golden/postprocess.json, tests/golden/postprocess_seeds.json).
 String / integer results: the bar is equality."""
-import importlib.util
 import json
 import os
 import sys
@@ -11,10 +10,11 @@ import pytest
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.join(ROOT, "tools"))
 
-from make_postprocess_goldens import chart  # noqa: E402
+from make_postprocess_goldens import SEEDS, chart, seed_case  # noqa: E402
 from mug_diffusion_b200 import postprocess as pp  # noqa: E402
 
 GOLD = json.load(open(os.path.join(ROOT, "tests", "golden", "postprocess.json")))
+SEED_GOLD = {g["case"]["seed"]: g for g in json.load(open(os.path.join(ROOT, "tests", "golden", "postprocess_seeds.json")))}
 
 
 @pytest.mark.parametrize("g", GOLD, ids=[f"seed{g['case']['seed']}" for g in GOLD])
@@ -37,16 +37,12 @@ def test_long_notes_are_never_moved_and_snapped_at_both_ends():
     assert len(grid) == 4 and all(l.split(",")[3] == o.split(",")[3] for l, o in zip(grid, lines))
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/mug/data/utils.py"), reason="reference tree not present")
-@pytest.mark.parametrize("seed", [11, 12, 13])
+@pytest.mark.parametrize("seed", SEEDS)
 def test_live_reference(seed):
-    spec = importlib.util.spec_from_file_location("ref_utils", "/root/reference/mug/data/utils.py")
-    ref = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(ref)
-    lines = chart(seed, 150 + 13.7 * seed % 140, 300 + seed, 150, div=4 if seed % 2 else 8, jack_ratio=0.15)
-    a = ref.remove_intractable_mania_mini_jacks(lines, verbose=False)
-    b = pp.remove_intractable_mania_mini_jacks(lines, verbose=False)
-    assert a == b
-    ga, bpm_a, off_a = ref.gridify(a, verbose=False)
+    """dejack -> gridify of a seeded chart against the reference's results for the same chart"""
+    g = SEED_GOLD[seed]
+    assert g["case"] == seed_case(seed)
+    b = pp.remove_intractable_mania_mini_jacks(chart(**g["case"]), verbose=False)
+    assert b == g["dejack"]
     gb, bpm_b, off_b = pp.gridify(b, verbose=False)
-    assert ga == gb and float(bpm_a) == float(bpm_b) and float(off_a) == float(off_b)
+    assert gb == g["grid"] and float(bpm_b) == g["bpm"] and float(off_b) == g["offset"]

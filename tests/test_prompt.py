@@ -1,6 +1,6 @@
 """Prompt path (SURVEY 8f N3): feature dict -> embedding ids -> [B,128,21] conditioning.
 CPU: the oracle restatement and the product's host function against ids produced by the UNMODIFIED reference
-(tests/golden/prompt.json, tools/make_goldens.py --only prompt), and against the live reference where its tree exists.
+(tests/golden/prompt.json, tools/make_goldens.py --only prompt; tests/golden/prompt_random.json, --only prompt_random).
 GPU: the gather kernel behind ``model.model.cond_stage_model`` bit-exact against the reference embedder's output."""
 import json
 import os
@@ -17,15 +17,7 @@ import golden_cases as gc  # noqa: E402
 from mug_diffusion_b200 import prompt as P  # noqa: E402
 from oracle import mug_oracle as orc  # noqa: E402
 
-REF = os.environ.get("MUG_REFERENCE_ROOT", "/root/reference")
-
-# a spec that exercises what the shipped yaml does not: count > 1 and non-integer bin edges
-SPEC_COUNT = [
-    {"name": "a", "type": "numeric", "min": 0.5, "max": 2.0, "interval": 0.25, "count": 3},
-    {"name": "b", "type": "category", "category": ["x", "y"], "count": 2},
-    {"name": "c", "type": "bool"},
-    {"name": "d", "type": "numeric", "min": -3, "max": 3, "interval": 1},
-]
+SPEC_COUNT = gc.PROMPT_SPEC_COUNT
 
 
 @pytest.fixture(scope="module")
@@ -65,28 +57,17 @@ def test_oracle_embed_matches_reference_golden(gold, golden_dir):
     assert torch.equal(orc.prompt_embed(g["table"], ids), g["out"])
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "mug")), reason="reference tree not present")
-def test_ids_match_live_reference_on_random_dicts(gold):
-    sys.path.insert(0, os.path.join(ROOT, "tools"))
-    import ref_shim
-    ref_shim.install_shims()
-    from mug.util import count_beatmap_features, feature_dict_to_embedding_ids
+def test_ids_match_live_reference_on_random_dicts(gold, golden_dir):
+    """300 seeded random dicts per spec against the ids the reference's feature_dict_to_embedding_ids gave them"""
+    cases = json.load(open(os.path.join(golden_dir, "prompt_random.json")))
     rnd = random.Random(5)
-    for spec in (gold["spec"], SPEC_COUNT):
-        assert P.count_beatmap_features(spec) == count_beatmap_features(spec)
-        for _ in range(300):
-            d = {}
-            for x in spec:
-                if rnd.random() < 0.4:
-                    continue
-                if x["type"] == "numeric":
-                    span = x["max"] - x["min"]
-                    d[x["name"]] = rnd.choice([x["min"] - 1, x["max"] + 1, x["min"] + span * rnd.random(), x["min"], x["max"]])
-                elif x["type"] == "bool":
-                    d[x["name"]] = rnd.choice([True, False, 0, 1])
-                else:
-                    d[x["name"]] = rnd.choice(x["category"])
-            want = feature_dict_to_embedding_ids(d, spec)
+    assert len(cases) == 2
+    for spec, case in zip((gold["spec"], SPEC_COUNT), cases):
+        assert case["spec"] == spec
+        dicts = gc.random_feature_dicts(spec, 300, rnd)
+        assert dicts == case["dicts"]
+        assert P.count_beatmap_features(spec) == case["n_embed"]
+        for d, want in zip(dicts, case["ids"]):
             assert P.feature_dict_to_embedding_ids(d, spec) == want
             assert orc.feature_ids(d, spec) == want
 

@@ -2,7 +2,7 @@
 tools/ref_shim.py) on the seeded synthetic weights/inputs of mug_diffusion_b200.synth.
 
 Run in the build container only (the GPU box has no /root/reference):
-    python tools/make_goldens.py [--only blocks|unet|ddim]
+    python tools/make_goldens.py [--only blocks|unet|ddim|s4len|wave|notes|prompt|prompt_random|refmodel]
 """
 import argparse
 import os
@@ -162,6 +162,45 @@ def make_prompt():
     print("prompt:", len(ids), "dicts,", len(ids[0]), "slots, table", tuple(emb.embedding.weight.shape))
 
 
+def make_prompt_random():
+    """The reference's count_beatmap_features and feature_dict_to_embedding_ids on 300 seeded random feature dicts for the
+    shipped spec (from prompt.json) and for a spec with count > 1 slots."""
+    import json
+    import random
+    ref_shim.install_shims()
+    from mug.util import count_beatmap_features, feature_dict_to_embedding_ids
+    rnd = random.Random(5)
+    out = []
+    for spec in (json.load(open(os.path.join(GOLD, "prompt.json")))["spec"], gc.PROMPT_SPEC_COUNT):
+        dicts = gc.random_feature_dicts(spec, 300, rnd)
+        out.append(dict(spec=spec, n_embed=count_beatmap_features(spec), dicts=dicts,
+                        ids=[feature_dict_to_embedding_ids(d, spec) for d in dicts]))
+    with open(os.path.join(GOLD, "prompt_random.json"), "w") as f:
+        json.dump(out, f)
+    print("wrote prompt_random.json", [len(c["dicts"]) for c in out])
+
+
+def make_reference_model():
+    """What MugDiffusionB200.config_from_reference reads off a reference DDPM built from the shipped yaml: the module
+    attributes and the name and shape of every state_dict entry."""
+    import json
+    model, _ = ref_shim.load_reference_model()
+    unet, fs = model.model.unet_model, model.model.first_stage_model
+    out = dict(
+        ddpm=dict(z_channels=int(model.z_channels), num_timesteps=int(model.num_timesteps),
+                  linear_start=float(model.linear_start), linear_end=float(model.linear_end)),
+        unet={a: (list(getattr(unet, a)) if isinstance(getattr(unet, a), (list, tuple)) else int(getattr(unet, a)))
+              for a in ("in_channels", "model_channels", "out_channels", "num_res_blocks", "attention_resolutions",
+                        "channel_mult", "num_heads")},
+        first_stage=dict(scale=float(fs.scale)),
+        decoder=dict(num_resolutions=int(fs.decoder.num_resolutions), num_res_blocks=int(fs.decoder.num_res_blocks),
+                     norm_out_num_groups=int(fs.decoder.norm_out.num_groups)),
+        state_dict={k: list(v.shape) for k, v in model.state_dict().items()})
+    with open(os.path.join(GOLD, "ref_model.json"), "w") as f:
+        json.dump(out, f)
+    print("wrote ref_model.json:", len(out["state_dict"]), "state_dict entries")
+
+
 def make_hit_objects():
     """OsuManiaConvertor.array_to_objects of the UNMODIFIED reference on the golden decoder logits (and on a synthetic
     logit array that exercises long notes running to the last frame, back-to-back starts and clipped offsets)."""
@@ -202,5 +241,9 @@ if __name__ == "__main__":
         make_hit_objects()
     if a.only in (None, "prompt"):
         make_prompt()
+    if a.only in (None, "prompt_random"):
+        make_prompt_random()
+    if a.only in (None, "refmodel"):
+        make_reference_model()
 
 

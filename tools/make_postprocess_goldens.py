@@ -1,5 +1,5 @@
 """Golden vectors for mug_diffusion_b200/postprocess.py from the UNMODIFIED reference (mug/data/utils.py), run in this container:
-    python tools/make_postprocess_goldens.py        -> tests/golden/postprocess.json
+    python tools/make_postprocess_goldens.py        -> tests/golden/postprocess.json, tests/golden/postprocess_seeds.json
 Synthetic charts (seeded): notes on a 1/4 or 1/8 grid of a known bpm/offset with jitter, chords, long notes and deliberate mini-jacks."""
 import importlib.util
 import json
@@ -38,6 +38,12 @@ def chart(seed, bpm, offset, n, div=4, jitter=3.0, ln_ratio=0.15, jack_ratio=0.0
 CASES = [dict(seed=1, bpm=187.3, offset=412, n=260), dict(seed=2, bpm=240.0, offset=1033, n=400, div=8, jitter=2.0),
          dict(seed=3, bpm=152.5, offset=95, n=120, jitter=4.0, ln_ratio=0.3), dict(seed=4, bpm=299.0, offset=2500, n=300, jack_ratio=0.2),
          dict(seed=5, bpm=175.0, offset=0, n=40, jitter=0.0, ln_ratio=0.0)]
+SEEDS = [11, 12, 13]
+
+
+def seed_case(seed):
+    """a denser-jack chart whose bpm, offset and grid follow from the seed"""
+    return dict(seed=seed, bpm=150 + 13.7 * seed % 140, offset=300 + seed, n=150, div=4 if seed % 2 else 8, jack_ratio=0.15)
 
 
 def main():
@@ -53,6 +59,13 @@ def main():
         out.append(dict(case=c, n_in=len(lines), dejack=dejack, grid=grid, bpm=float(bpm), offset=float(off), dejack_after_grid=dejack2))
         print(c, len(lines), "->", len(dejack), "->", len(dejack2), "bpm", bpm, "offset", off)
     json.dump(out, open(os.path.join(ROOT, "tests", "golden", "postprocess.json"), "w"))
+    out = []
+    for seed in SEEDS:
+        c = seed_case(seed)
+        dejack = ref.remove_intractable_mania_mini_jacks(chart(**c), verbose=False)
+        grid, bpm, off = ref.gridify(dejack, verbose=False)
+        out.append(dict(case=c, dejack=dejack, grid=grid, bpm=float(bpm), offset=float(off)))
+    json.dump(out, open(os.path.join(ROOT, "tests", "golden", "postprocess_seeds.json"), "w"))
 
 
 if __name__ == "__main__":
