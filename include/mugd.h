@@ -28,7 +28,7 @@
 extern "C" {
 #endif
 
-#define MUGD_ABI_VERSION 12
+#define MUGD_ABI_VERSION 13
 
 typedef struct mugd_handle mugd_handle;   /* one device + scratch state            */
 typedef struct mugd_plan mugd_plan;       /* validated launch plan (+ CUDA graph)  */
@@ -72,6 +72,10 @@ enum mugd_gate { MUGD_GATE_NONE = 0, MUGD_GATE_GEGLU = 1 /* a*gelu(g), attention
                  MUGD_GATE_GLU = 2 /* a*sigmoid(g), s4.py:191-192,1536 */ };
 enum mugd_gemm_impl { MUGD_GEMM_AUTO = 0, MUGD_GEMM_SIMT = 1 /* exact fp32 FMA */,
                       MUGD_GEMM_TC = 2 /* tcgen05 3xTF32 split, fp32 accumulate in TMEM */ };
+/* tile variant of the tensor-core GEMM (mugd_gemm.tc_variant): AUTO = the planner's cost model; the others force a variant where
+ * the shape allows it (a tile wider than N falls back to the 128- or 64-wide tile) */
+enum mugd_tc_variant { MUGD_TC_AUTO = 0, MUGD_TC_N64 = 1, MUGD_TC_N128 = 2, MUGD_TC_N256 = 3,
+                       MUGD_TC_N128_2CTA = 4 /* 128 wide, two CTAs per SM walking a tile list */ };
 
 typedef struct mugd_gemm {
     const float* A;  int64_t lda;          /* [B*Lin, K] activations                                       */
@@ -89,17 +93,16 @@ typedef struct mugd_gemm {
     int32_t taps, conv_mode, Lin, Lout;
     int32_t act, gate, impl;
     int32_t split_k;                       /* tensor-core path: 0 = auto, >0 forces the K split            */
-    int32_t n_counters;                    /* entries available in `counters`                              */
     int32_t tap_shift;                     /* MUGD_CONV_TAPS: source row of tap t is l + (t + tap_shift) * dilation */
     int32_t tap_dilation;                  /* MUGD_CONV_TAPS: 0/1 = dense taps; d = dilated conv (wave.py:425-433)  */
     void* workspace; int64_t workspace_bytes; /* split-K partial tiles (see mugd_gemm_tc_query)            */
-    int32_t* counters;                     /* unused since ABI 8 (kept for layout stability)               */
     /* optional SECOND activation source: K2 more channels read at the output row itself (a 1x1 term), weights in columns
      * taps*K .. taps*K+K2 of every W row.  One GEMM then computes  conv3(A) + conv1(A2):  out_layers conv + skip_connection
      * of a TimestepResBlock (unet.py:187-193,237-239), and  proj_out(ff.net.2(ff) + h) = (Wp Wf) ff + Wp h  of the transformer
      * block (attention.py:57-65,194-199) with the packer-composed weight.  NULL / 0 = single source. */
     const float* A2; int64_t lda2;         /* [B*Lout, K2]                                                 */
-    int32_t K2; int32_t reserved_;
+    int32_t K2;
+    int32_t tc_variant;                    /* tensor-core path: enum mugd_tc_variant, 0 = auto             */
     /* Row moments of the OUTPUT for a LayerNorm that follows (tensor-core path, act == gate == NONE only): while the tile is stored,
      * row_moments[m*2 + {0,1}] += {sum, sum of squares} of the columns of output row m (fp64 atomics; the plan zeroes the buffer at
      * the start of every evaluation).  Round 2 also built GroupNorm-moment sinks + a single-pass apply kernel; they lost at every batch
@@ -207,7 +210,6 @@ int  mugd_create(int device, mugd_handle** out);           /* MUGD_ERR_NO_DEVICE
 void mugd_destroy(mugd_handle* h);
 int  mugd_device_info(mugd_handle* h, int32_t* sm_count, int32_t* cc_major, int32_t* cc_minor);
 int  mugd_set_gemm_impl(mugd_handle* h, int impl);         /* default for ops with impl == AUTO         */
-int  mugd_set_pdl(int enabled);                            /* programmatic launch edges (default on; process-wide A/B switch) */
 
 /* ---- single op (parity tests call every kernel through this) ---------------------------------- */
 int  mugd_op_run(mugd_handle* h, const mugd_op* op, void* stream);
@@ -254,7 +256,7 @@ int  mugd_s4_kernel_gen(mugd_handle* h,
                         void* stream);
 
 /* ---- tensor-core GEMM planning: is this GEMM taken by the tcgen05 kernel, with which K split, and how much
- * split-K workspace / how many tile counters does it need (the host allocates them once per plan) ------ */
+ * split-K workspace does it need (the host allocates it once per plan) ------ */
 int  mugd_gemm_tc_query(mugd_handle* h, const mugd_gemm* g, int32_t sm_count, int32_t* supported, int32_t* splits,
                         int64_t* workspace_bytes, int32_t* n_tiles);
 /* which kernel variant the planner picks for this GEMM on a machine with sm_count SMs: tile width (64 / 128 / 256; 0 = not taken by the
@@ -271,19 +273,8 @@ int  mugd_set_tc_single_pass_tf32(mugd_handle* h, int enabled);
  * (the referee of the parity tests).  Replaces the einsum/softmax body of CrossAttention.forward, attention.py:99-121 */
 int  mugd_set_attention_impl(mugd_handle* h, int impl);
 
-/* ---- measurement aids (process-wide, not needed in production) -------------------------------------
- * planner cost constants of the tensor-core GEMM (us per 32-deep k-step of a 128- and a 256-column tile, us per split-K
- * round trip, fixed us of the two-CTAs-per-SM variant); values <= 0 keep the current one.  For tuning sweeps (tools/). */
-int  mugd_debug_set_tc_cost(float kstep128_us, float kstep256_us, float split_us, float two_cta_fixed_us);
-
-/* force the tensor-core tile variant (64, 128, 256 columns, or 130 = 128 columns built for two CTAs per SM) where legal; 0 = cost model */
-int  mugd_debug_set_tc_tile_n(int bn);
-
-/* CTA (0,0,0) of the tensor-core attention kernel dumps 40 floats per query row of its first key tile
- * (raw logits, O tile, running max / sum, first operand words) into buf[128*40]; NULL switches it off */
-int  mugd_debug_set_attention_dump(float* buf);
-
-/* builds with -DMUGD_TC_TIMELINE only (tools/build_variant.py): CTA (0,0,0) of every tensor-core GEMM launch writes
+/* ---- measurement aid ------------------------------------------------------------------------------------
+ * builds with -DMUGD_TC_TIMELINE only (tools/build_variant.py): CTA (0,0,0) of every tensor-core GEMM launch writes
  * %globaltimer stamps into the device buffer (tools/gemm_timeline.py); otherwise returns MUGD_ERR_INVALID */
 int  mugd_debug_set_tc_timing(long long* device_buf);
 

@@ -75,7 +75,7 @@ def export_bundle(model, inp: Dict[str, torch.Tensor], S: int, scale: float, out
         # ---- regions: every device allocation a plan may point into ----
         tensors: Dict[str, torch.Tensor] = dict(weights=eng.weights, weights_lo=eng.weights_lo, arena=sess.arena_t, emb_table=sess.emb_table, temb=sess.temb,
                                                 emb_h1=sess.emb_h1, emb_h2=sess.emb_h2, step=sess.step, coef=sess.coef, ctx=sess.ctx,
-                                                tc_ws=eng.tc_ws, tc_counters=eng.tc_counters, dec_arena=dec.arena_t)
+                                                tc_ws=eng.tc_ws, dec_arena=dec.arena_t)
         for i, t in enumerate(sess.ctx_kv):
             tensors[f"ctx_kv{i}"] = t
         for i, (_, t) in enumerate(sorted(sess.s4_kt.items())):

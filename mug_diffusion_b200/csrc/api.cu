@@ -9,9 +9,6 @@
 namespace mugd {
 
 static thread_local char g_err[1024] = "";
-// Programmatic launch edges with the implicit (grid-completion) trigger: graph edge 0.57 vs 0.69 us, 3.97 vs 4.02 ms/step.  This is a
-// launch attribute without numerical effect; it is process-wide because launch_k() has no handle (mugd_set_pdl is an A/B switch).
-bool g_use_pdl = true;
 
 void set_error(const char* fmt, ...) {
     va_list ap;
@@ -87,12 +84,19 @@ int mugd_create(int device, mugd_handle** out) {
         return MUGD_ERR_NO_DEVICE;
     }
     MUGD_CHECK_CUDA(cudaSetDevice(device));
+    DeviceInfo dev;
+    dev.device = device;
+    dev.sm_count = prop.multiProcessorCount;
+    dev.cc_major = prop.major;
+    dev.cc_minor = prop.minor;
+    dev.max_smem_optin = (int)prop.sharedMemPerBlockOptin;
+    int rc = configure_gemm_tc_kernels(dev);
+    if (rc == MUGD_OK) rc = configure_attention_kernels(dev);
+    if (rc == MUGD_OK) rc = configure_attention_tc_kernels(dev);
+    if (rc == MUGD_OK) rc = configure_s4_kernels(dev);
+    if (rc != MUGD_OK) return rc;
     mugd_handle* h = new mugd_handle();
-    h->dev.device = device;
-    h->dev.sm_count = prop.multiProcessorCount;
-    h->dev.cc_major = prop.major;
-    h->dev.cc_minor = prop.minor;
-    h->dev.max_smem_optin = (int)prop.sharedMemPerBlockOptin;
+    h->dev = dev;
     *out = h;
     return MUGD_OK;
 }
@@ -123,11 +127,6 @@ int mugd_set_tc_single_pass_tf32(mugd_handle* h, int enabled) {
 int mugd_set_attention_impl(mugd_handle* h, int impl) {
     MUGD_REQUIRE(h, "null handle");
     h->dev.attention_impl = impl ? 1 : 0;
-    return MUGD_OK;
-}
-
-int mugd_set_pdl(int enabled) {
-    g_use_pdl = enabled != 0;
     return MUGD_OK;
 }
 

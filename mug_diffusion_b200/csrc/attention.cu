@@ -46,7 +46,6 @@ attention_kernel(const mugd_attention a) {
     const int P = a.pos_max, NT = 2 * P + 1;
     float* cg = rel + NT;
 
-    pdl_trigger();
     pdl_wait();
     const int tid = threadIdx.x, tx = tid & 15, ty = tid >> 4;
     const int b = blockIdx.z, h = blockIdx.y;
@@ -168,15 +167,20 @@ attention_kernel(const mugd_attention a) {
 }
 
 template <int D>
-static int attention_launch(const mugd_attention& a, cudaStream_t st) {
+static int attention_launch(const DeviceInfo& dev, const mugd_attention& a, cudaStream_t st) {
     const size_t bytes = sizeof(float) * (AttSmem<D>::FLOATS + 2 * (2 * a.pos_max + 1));
-    static size_t configured = 0;
-    if (bytes > configured) {
-        MUGD_CHECK_CUDA(cudaFuncSetAttribute(attention_kernel<D>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
-        configured = bytes;
-    }
+    MUGD_REQUIRE(bytes <= (size_t)dev.max_smem_optin, "attention: pos_max=%d needs %zu B of shared memory (max %d)", a.pos_max, bytes,
+                 dev.max_smem_optin);
     dim3 grid((a.Lq + AT_BQ - 1) / AT_BQ, a.H, a.B);
     MUGD_CHECK_CUDA(launch_k(attention_kernel<D>, grid, dim3(AT_THREADS), bytes, st, a));
+    return MUGD_OK;
+}
+
+// the byte count grows with pos_max: allow what the device allows, the launcher checks each launch against it
+int configure_attention_kernels(const DeviceInfo& dev) {
+    MUGD_CHECK_CUDA(cudaFuncSetAttribute(attention_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, dev.max_smem_optin));
+    MUGD_CHECK_CUDA(cudaFuncSetAttribute(attention_kernel<48>, cudaFuncAttributeMaxDynamicSharedMemorySize, dev.max_smem_optin));
+    MUGD_CHECK_CUDA(cudaFuncSetAttribute(attention_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, dev.max_smem_optin));
     return MUGD_OK;
 }
 
@@ -326,7 +330,7 @@ int launch_attention(const DeviceInfo& dev, const mugd_attention& a, cudaStream_
     if (dev.attention_impl == 1 && a.Lk <= 32 && a.D >= 48)
         rc = (a.D == 48) ? attention_smallk_launch<48>(a, st) : attention_smallk_launch<64>(a, st);
     else if (dev.attention_impl == 1) rc = launch_attention_tc(dev, a, st);
-    else rc = (a.D == 32) ? attention_launch<32>(a, st) : (a.D == 48) ? attention_launch<48>(a, st) : attention_launch<64>(a, st);
+    else rc = (a.D == 32) ? attention_launch<32>(dev, a, st) : (a.D == 48) ? attention_launch<48>(dev, a, st) : attention_launch<64>(dev, a, st);
     if (rc != MUGD_OK) return rc;
     if (launches) *launches += 1;
     return MUGD_OK;

@@ -141,7 +141,7 @@ struct Smem {
 
 template <int D>
 __global__ void __launch_bounds__(THREADS, 1)
-attention_tc_kernel(const __grid_constant__ CUtensorMap tmK, const __grid_constant__ CUtensorMap tmV, const mugd_attention a, float* dbg) {
+attention_tc_kernel(const __grid_constant__ CUtensorMap tmK, const __grid_constant__ CUtensorMap tmV, const mugd_attention a) {
     using S = Smem<D>;
     constexpr int HC = D / 2;                               // Q / O columns owned by one thread of a row pair
     constexpr int STAGES = S::STAGES;
@@ -165,7 +165,6 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tmK, const __grid_consta
     const int b = blockIdx.z, h = blockIdx.y, q0 = blockIdx.x * BQ;
     const int ntiles = (a.Lk + BKV - 1) / BKV;
 
-    pdl_trigger();
     if (tid == 0) {
         for (int s = 0; s < STAGES; ++s) mbar_init(bar_full(s), 1);
         mbar_init(bar_s, 1);
@@ -306,12 +305,6 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tmK, const __grid_consta
                 tmem_ld8(lane_addr + TM_S + c0, v);
                 tmem_ld8(lane_addr + TM_S + c0 + 8, v + 8);
                 tmem_wait_ld();
-                if (dbg && blockIdx.x == 0 && blockIdx.y == 0 && blockIdx.z == 0 && t == 0 && g == 0 && ci == 0) {
-                    for (int j = 0; j < 16; ++j) dbg[r * 40 + j] = v[j];
-                    const float4 vv = lds_f4(vt_hi + (r & 63) * 128), kv = lds_f4(k_hi(s) + r * 128);
-                    dbg[r * 40 + 26] = vv.x; dbg[r * 40 + 27] = vv.y; dbg[r * 40 + 28] = vv.z; dbg[r * 40 + 29] = vv.w;
-                    dbg[r * 40 + 30] = kv.x; dbg[r * 40 + 31] = kv.y; dbg[r * 40 + 32] = kv.z; dbg[r * 40 + 33] = kv.w;
-                }
 #pragma unroll
                 for (int j = 0; j < 16; ++j) {
                     const int kj = j0 + c0 + j;
@@ -383,10 +376,6 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tmK, const __grid_consta
             float ot[8];
             tmem_ld8(lane_addr + TM_O + g * HC + c * 8, ot);
             tmem_wait_ld();
-            if (dbg && blockIdx.x == 0 && blockIdx.y == 0 && blockIdx.z == 0 && t == 0 && g == 0 && c == 0) {
-                for (int j = 0; j < 8; ++j) dbg[r * 40 + 16 + j] = ot[j];
-                dbg[r * 40 + 24] = m_i; dbg[r * 40 + 25] = l_i;
-            }
 #pragma unroll
             for (int j = 0; j < 8; ++j) o[c * 8 + j] = fmaf(o[c * 8 + j], corr, ot[j]);
         }
@@ -408,21 +397,6 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tmK, const __grid_consta
     }
 }
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-static EncodeTiledFn get_encode() {
-    static EncodeTiledFn fn = nullptr;
-    if (!fn) {
-        void* p = nullptr;
-        cudaDriverEntryPointQueryResult qr;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qr) == cudaSuccess && qr == cudaDriverEntryPointSuccess)
-            fn = (EncodeTiledFn)p;
-    }
-    return fn;
-}
-
 // (channel, key, sample) view of a [B*Lk, ld] row-major buffer whose first H*D columns are the head slices
 static int encode_kv(EncodeTiledFn enc, CUtensorMap* tm, const float* p, int64_t ld, int cols, int Lk, int B) {
     cuuint64_t dims[3] = {(cuuint64_t)cols, (cuuint64_t)Lk, (cuuint64_t)B};
@@ -436,10 +410,8 @@ static int encode_kv(EncodeTiledFn enc, CUtensorMap* tm, const float* p, int64_t
     return MUGD_OK;
 }
 
-static float* g_dbg = nullptr;      // debugging aid: CTA (0,0,0) dumps 40 floats per query row of its first key tile
-
 template <int D>
-static int launch(const mugd_attention& a, cudaStream_t st) {
+static int launch(const DeviceInfo& dev, const mugd_attention& a, cudaStream_t st) {
     EncodeTiledFn enc = get_encode();
     MUGD_REQUIRE(enc != nullptr, "attention_tc: cuTensorMapEncodeTiled entry point not available");
     CUtensorMap tmK, tmV;
@@ -448,25 +420,25 @@ static int launch(const mugd_attention& a, cudaStream_t st) {
     rc = encode_kv(enc, &tmV, a.v, a.ldv, a.H * D, a.Lk, a.B);
     if (rc != MUGD_OK) return rc;
     const size_t bytes = Smem<D>::total(a.pos_max);
-    static size_t configured = 0;
-    if (bytes > configured) {
-        MUGD_CHECK_CUDA(cudaFuncSetAttribute(attention_tc_kernel<D>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
-        configured = bytes;
-    }
+    MUGD_REQUIRE(bytes <= (size_t)dev.max_smem_optin, "attention_tc: pos_max=%d needs %zu B of shared memory (max %d)", a.pos_max, bytes,
+                 dev.max_smem_optin);
     dim3 grid((a.Lq + BQ - 1) / BQ, a.H, a.B);
-    MUGD_CHECK_CUDA(launch_k(attention_tc_kernel<D>, grid, dim3(THREADS), bytes, st, tmK, tmV, a, g_dbg));
+    MUGD_CHECK_CUDA(launch_k(attention_tc_kernel<D>, grid, dim3(THREADS), bytes, st, tmK, tmV, a));
     return MUGD_OK;
 }
 
 }  // namespace atc
 
-int launch_attention_tc(const DeviceInfo&, const mugd_attention& a, cudaStream_t st) {
-    return (a.D == 32) ? atc::launch<32>(a, st) : (a.D == 48) ? atc::launch<48>(a, st) : atc::launch<64>(a, st);
+// the byte count grows with pos_max: allow what the device allows, the launcher checks each launch against it
+int configure_attention_tc_kernels(const DeviceInfo& dev) {
+    MUGD_CHECK_CUDA(cudaFuncSetAttribute(atc::attention_tc_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, dev.max_smem_optin));
+    MUGD_CHECK_CUDA(cudaFuncSetAttribute(atc::attention_tc_kernel<48>, cudaFuncAttributeMaxDynamicSharedMemorySize, dev.max_smem_optin));
+    MUGD_CHECK_CUDA(cudaFuncSetAttribute(atc::attention_tc_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, dev.max_smem_optin));
+    return MUGD_OK;
+}
+
+int launch_attention_tc(const DeviceInfo& dev, const mugd_attention& a, cudaStream_t st) {
+    return (a.D == 32) ? atc::launch<32>(dev, a, st) : (a.D == 48) ? atc::launch<48>(dev, a, st) : atc::launch<64>(dev, a, st);
 }
 
 }  // namespace mugd
-
-extern "C" int mugd_debug_set_attention_dump(float* buf) {
-    mugd::atc::g_dbg = buf;
-    return MUGD_OK;
-}

@@ -1,5 +1,6 @@
 // Shared host/device helpers of libmugd (sm_100a only).
 #pragma once
+#include <cuda.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
@@ -62,12 +63,17 @@ int launch_tf32_split(const DeviceInfo& dev, const mugd_tf32_split& s, cudaStrea
 int launch_gemm_tc(const DeviceInfo& dev, const mugd_gemm& g, cudaStream_t st, int* launches);
 bool gemm_tc_supported(const mugd_gemm& g);
 
-// Programmatic dependent launch (PDL): every hot-path kernel is launched with the programmatic-stream-serialization
-// attribute, signals `launch_dependents` at entry and executes `griddepcontrol.wait` before its first global-memory
-// access.  The next kernel's launch latency and prologue (block scheduling, barrier init, TMEM allocation,
-// tensor-map fetch) then overlap the tail of the current one; data hazards are unchanged because the wait
-// only returns when the prerequisite grid has completed and flushed.
-extern bool g_use_pdl;
+// Kernel attributes are per device: mugd_create sets them on its device for every instantiation the launchers can pick (dynamic
+// shared memory above the 48 KB default, carveout).
+int configure_gemm_tc_kernels(const DeviceInfo& dev);
+int configure_attention_kernels(const DeviceInfo& dev);
+int configure_attention_tc_kernels(const DeviceInfo& dev);
+int configure_s4_kernels(const DeviceInfo& dev);
+
+// Programmatic dependent launch (PDL): launch_k always sets the programmatic-stream-serialization attribute, and every kernel it
+// launches executes `griddepcontrol.wait` before its first global-memory access.  The next kernel's launch latency and prologue
+// (block scheduling, barrier init, TMEM allocation, tensor-map fetch) then overlap the tail of the current one; data hazards
+// are unchanged because the wait only returns when the prerequisite grid has completed and flushed.
 
 #ifdef __CUDACC__
 template <typename... KArgs, typename... Args>
@@ -81,13 +87,12 @@ inline cudaError_t launch_k(void (*kernel)(KArgs...), dim3 grid, dim3 block, siz
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
-    cfg.numAttrs = g_use_pdl ? 1 : 0;
+    cfg.numAttrs = 1;
     return cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...);
 }
 // No kernel signals launch_dependents explicitly: the trigger is implicit at grid completion, so PDL only overlaps the dependent's
 // launch with this grid's memory flush (graph edge 0.57 us instead of 0.69 us, tools/experiments/sync_probe.cu).  Explicit triggers
 // (at entry, in the short kernels only, after the GEMM main loop) were measured slower in round 1 (DESIGN.md 4) and removed.
-__device__ __forceinline__ void pdl_trigger() {}
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 
 // ---- device helpers ---------------------------------------------------------------------------
@@ -113,5 +118,21 @@ __device__ __forceinline__ float warp_max(float v) {
 #endif
 
 inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
+
+// cuTensorMapEncodeTiled of the driver the runtime runs on (tensor maps of the tcgen05 GEMM and attention); null if unavailable
+typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
+                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
+                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+
+inline EncodeTiledFn get_encode() {
+    static EncodeTiledFn fn = nullptr;
+    if (!fn) {
+        void* p = nullptr;
+        cudaDriverEntryPointQueryResult qr;
+        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qr) == cudaSuccess && qr == cudaDriverEntryPointSuccess)
+            fn = (EncodeTiledFn)p;
+    }
+    return fn;
+}
 
 }  // namespace mugd

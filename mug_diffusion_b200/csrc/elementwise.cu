@@ -12,7 +12,6 @@ namespace mugd {
 // ATen ops (no FMA contraction), so given identical eps the update is bit-identical.
 __global__ void __launch_bounds__(256)
 ddim_update_kernel(const mugd_ddim_update d) {
-    pdl_trigger();
     pdl_wait();
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= d.n) return;
@@ -49,7 +48,6 @@ int launch_ddim_update(const DeviceInfo&, const mugd_ddim_update& d, cudaStream_
 __global__ void __launch_bounds__(256)
 transpose_kernel(const mugd_transpose t) {
     __shared__ float tile[32][33];
-    pdl_trigger();
     pdl_wait();
     const int b = blockIdx.z;
     const int c0 = blockIdx.y * 32, l0 = blockIdx.x * 32;
@@ -98,7 +96,6 @@ int launch_transpose(const DeviceInfo&, const mugd_transpose& t, cudaStream_t st
 
 __global__ void __launch_bounds__(256)
 copy2d_kernel(const mugd_copy2d c) {
-    pdl_trigger();
     pdl_wait();
     const int q = c.cols >> 2;
     const int64_t total = (int64_t)c.rows * q;
@@ -123,6 +120,7 @@ int launch_copy2d(const DeviceInfo& dev, const mugd_copy2d& c, cudaStream_t st, 
 // weight preprocessing for the 3xTF32 GEMM: hi over w, lo beside it (same roundings as the converter warps apply to activations)
 __global__ void __launch_bounds__(256)
 tf32_split_kernel(float* __restrict__ w_hi, float* __restrict__ lo, int64_t n4) {
+    pdl_wait();
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (int64_t)gridDim.x * blockDim.x) {
         const float4 w = ld_f4(w_hi + i * 4);
         float4 h, l;
@@ -147,7 +145,6 @@ int launch_tf32_split(const DeviceInfo& dev, const mugd_tf32_split& s, cudaStrea
 }
 
 __global__ void step_advance_kernel(int32_t* step) {
-    pdl_trigger();
     pdl_wait();
     *step += 1;
 }
@@ -165,7 +162,6 @@ int launch_step_advance(const DeviceInfo&, const mugd_step_advance& a, cudaStrea
 // compacted with a ballot/prefix scan so the output is ordered by frame like the reference's np.where loop.
 __global__ void __launch_bounds__(256)
 notes_kernel(const mugd_notes n) {
-    pdl_trigger();
     pdl_wait();
     const int c = blockIdx.x, b = blockIdx.y;
     const int K = n.K, T = n.T;
@@ -229,7 +225,6 @@ int launch_notes(const DeviceInfo&, const mugd_notes& n, cudaStream_t st, int* l
 // sample: 10 KB per request, latency only).
 __global__ void __launch_bounds__(128)
 embed_kernel(const mugd_embed e) {
-    pdl_trigger();
     pdl_wait();
     const int f = blockIdx.x, b = blockIdx.y;
     const int id = e.ids[b * e.F + f];

@@ -50,7 +50,6 @@ gemm_simt_kernel(const GemmParams p) {
     __shared__ __align__(16) float As[2][SG_BK][SA];
     __shared__ __align__(16) float Ws[2][SG_BK][SW];
 
-    pdl_trigger();
     pdl_wait();
     const mugd_gemm& g = p.g;
     const int tid = threadIdx.x;

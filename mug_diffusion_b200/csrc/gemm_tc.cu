@@ -67,12 +67,12 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         const int n_tiles = p.gx * p.gy;
         int done = 0;
         for (int tile = (int)blockIdx.x; tile < n_tiles; tile += (int)gridDim.x, ++done) {
-            gemm_tc_tile<BN, true, EPI, OCC>(&tmA, &tmA1, &tmA2, &tmB, &tmWhi, &tmWlo, p, tile % p.gx, tile / p.gx, 0, base, tmem_base,
-                                             done * p.hot.total_it, (uint32_t)done & 1u);
+            gemm_tc_tile<BN, EPI, OCC>(&tmA, &tmA1, &tmA2, &tmB, &tmWhi, &tmWlo, p, tile % p.gx, tile / p.gx, 0, base, tmem_base,
+                                       done * p.hot.total_it, (uint32_t)done & 1u);
             __syncthreads();         // the staged tile has been read: the next tile's TMA may overwrite the pipeline buffers
         }
     } else {
-        gemm_tc_tile<BN, true, EPI, OCC>(&tmA, &tmA1, &tmA2, &tmB, &tmWhi, &tmWlo, p, blockIdx.x, blockIdx.y, blockIdx.z, base, tmem_base);
+        gemm_tc_tile<BN, EPI, OCC>(&tmA, &tmA1, &tmA2, &tmB, &tmWhi, &tmWlo, p, blockIdx.x, blockIdx.y, blockIdx.z, base, tmem_base);
     }
     // ---- teardown (all tcgen05.ld completed before the phase-2 barrier inside the tile function) ----
     __syncthreads();
@@ -93,35 +93,19 @@ gemm_tc_reduce_kernel(const __grid_constant__ TcParams p) {
 static long long* g_tc_dbg = nullptr;
 #endif
 // planner constants: us per k-step of a 128- / 256-wide tile (tools/bench_gemm.py), us per split-K round trip (workspace + reduce
-// launch).  The split cost was 4.0 in round 1; with the slimmer kernels of round 2 the sweep (tools/experiments/sweep_cost.sh:
-// 299 / 303 / 312 / 312 steps/s at 5.0 / 4.0 / 3.0 / 2.0) favours splitting a little more.  mugd_debug_set_tc_cost for sweeps
+// launch).  The split cost was 4.0 in round 1; with the slimmer kernels of round 2 a bench.py sweep of it (299 / 303 / 312 / 312
+// steps/s at 5.0 / 4.0 / 3.0 / 2.0) favours splitting a little more.
 // The two-CTAs-per-SM variant (TcSmem<128, 2>) is taken when its estimate -- tiles per SM x k-steps x the 128-wide k-step, two residents
-// sharing one tensor pipe -- beats the best single-resident estimate by more than g_tc_cost[3].  That constant is a CREDIT (negative):
+// sharing one tensor pipe -- beats the best single-resident estimate by more than k_tc_cost[3].  That constant is a CREDIT (negative):
 // the single-resident estimates carry 1.0 us of fill per wave because only their differences matter to the split decision, while a
 // wave really exposes ~7 us of prologue + accumulator drain that two residents hide behind each other's main loop.  Fitted on the
 // per-op tables of Beff = 64 / L = 512 and Beff = 16 / L = 992 (tools/compare_ops.py): every GEMM it picks was measured faster
 // (0.71-0.98x), the ones it leaves alone (fewer tiles than SMs, or long K with < 2 tiles per SM) were slower or even.
-static float g_tc_cost[4] = {0.55f, 0.9f, 3.0f, -6.5f};
-static int g_tc_force_bn = 0;        // experiments: 0 = cost model, 64 / 128 / 256 = force the tile width where legal
+constexpr float k_tc_cost[4] = {0.55f, 0.9f, 3.0f, -6.5f};
 
 // =====================================================================================================
 // host side
 // =====================================================================================================
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-static EncodeTiledFn get_encode() {
-    static EncodeTiledFn fn = nullptr;
-    if (!fn) {
-        void* p = nullptr;
-        cudaDriverEntryPointQueryResult qr;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qr) == cudaSuccess && qr == cudaDriverEntryPointSuccess)
-            fn = (EncodeTiledFn)p;
-    }
-    return fn;
-}
-
 static bool tc_shape_ok(const mugd_gemm& g) {
     if (!(g.conv_mode == MUGD_CONV_NONE || g.conv_mode == MUGD_CONV_SAME || g.conv_mode == MUGD_CONV_DOWN ||
           g.conv_mode == MUGD_CONV_TAPS)) return false;
@@ -176,24 +160,26 @@ TcGeometry tc_geometry(const mugd_gemm& g, int sm_count, int forced_split) {
     int splits = 1;
     float best = 1e30f;
     static const int cands[4] = {64, 128, 256, 130 /* 128 wide, two CTAs per SM */};
+    // a forced variant (mugd_gemm.tc_variant) in the same codes; 0 = cost model
+    const int force = (g.tc_variant >= MUGD_TC_N64 && g.tc_variant <= MUGD_TC_N128_2CTA) ? cands[g.tc_variant - MUGD_TC_N64] : 0;
     for (int cand = 0; cand < 4; ++cand) {
         const int code = cands[cand];
         const int bn = code == 130 ? 128 : code;
         const int occ = code == 130 ? 2 : 1;
         if (bn > 64 && g.N < bn) continue;
-        if (bn == 64 && g.N >= 128 && g_tc_force_bn != 64) continue;
-        if (g_tc_force_bn && code != g_tc_force_bn && !((g_tc_force_bn == 256 ? 256 : 128) > g.N && code == (g.N >= 128 ? 128 : 64))) continue;
+        if (bn == 64 && g.N >= 128 && force != 64) continue;
+        if (force && code != force && !((force == 256 ? 256 : 128) > g.N && code == (g.N >= 128 ? 128 : 64))) continue;
         const int gx = (g.N + bn - 1) / bn;
         const int tiles = gx * t.gy;
         if (occ == 2) {
             // two residents per SM share one tensor pipe: n tiles per SM back to back, one exposed prologue + epilogue
-            if (forced_split > 1 || (tiles <= sm_count && g_tc_force_bn != 130)) continue;
+            if (forced_split > 1 || (tiles <= sm_count && force != 130)) continue;
             const int n = (tiles + sm_count - 1) / sm_count;
-            const float est = g_tc_cost[3] + n * g_tc_cost[0] * t.total_it;
-            if (est < best - 0.25f || g_tc_force_bn == 130) { best = est; splits = 1; t.BN = 128; t.occ = 2; }
+            const float est = k_tc_cost[3] + n * k_tc_cost[0] * t.total_it;
+            if (est < best - 0.25f || force == 130) { best = est; splits = 1; t.BN = 128; t.occ = 2; }
             continue;
         }
-        const float kstep = bn == 256 ? g_tc_cost[1] : (bn == 128 ? g_tc_cost[0] : 0.4f);
+        const float kstep = bn == 256 ? k_tc_cost[1] : (bn == 128 ? k_tc_cost[0] : 0.4f);
         // 256-wide tiles only pay off unsplit (measured: l1/l2 FF1 and the B=64 convs gain 15-25 %, split cases lose)
         const int sp_max = forced_split > 0 ? forced_split : ((tiles < sm_count && bn != 256) ? 16 : 1);
         for (int sp = forced_split > 0 ? forced_split : 1; sp <= sp_max && sp <= t.total_it; ++sp) {
@@ -201,7 +187,7 @@ TcGeometry tc_geometry(const mugd_gemm& g, int sm_count, int forced_split) {
             if (forced_split <= 0 && sp > 1 && per < 2) break;
             if (forced_split <= 0 && sp > 1 && tiles * sp > 2 * sm_count) break;   // bounds the workspace: < 2*SMs partial tiles
             const int waves = (tiles * sp + sm_count - 1) / sm_count;
-            const float est = waves * (1.0f + kstep * per) + (sp > 1 ? g_tc_cost[2] : 0.0f);
+            const float est = waves * (1.0f + kstep * per) + (sp > 1 ? k_tc_cost[2] : 0.0f);
             if (est < best - 0.25f) { best = est; splits = sp; t.BN = bn; t.occ = 1; }
         }
     }
@@ -216,6 +202,7 @@ TcGeometry tc_geometry(const mugd_gemm& g, int sm_count, int forced_split) {
 
 int tc_plan(const DeviceInfo& dev, const mugd_gemm& g, TcPlanned* out) {
     MUGD_REQUIRE(gemm_tc_supported(g), "gemm_tc: unsupported shape/operands");
+    MUGD_REQUIRE(g.tc_variant >= MUGD_TC_AUTO && g.tc_variant <= MUGD_TC_N128_2CTA, "gemm_tc: tc_variant %d", g.tc_variant);
     {
         const int rc = tc_validate_fusions(g);
         if (rc != MUGD_OK) return rc;
@@ -304,11 +291,6 @@ static int tc_launch(const TcPlanned& pl, cudaStream_t st) {
     const TcParams& p = pl.p;
     if (p.splits > 1) {
         // the main kernel only writes partial tiles: it runs the smallest instantiation, the epilogue variant lives in the reduce
-        static bool configured = false;
-        if (!configured) {
-            MUGD_CHECK_CUDA(cudaFuncSetAttribute(gemm_tc_kernel<BN, TC_E_NONE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TcSmem<BN>::TOTAL));
-            configured = true;
-        }
         MUGD_CHECK_CUDA(launch_k(gemm_tc_kernel<BN, TC_E_NONE>, dim3(p.gx, p.gy, p.splits), dim3(TC_THREADS), TcSmem<BN>::TOTAL, st, pl.maps[0],
                                  pl.maps[1], pl.maps[2], pl.maps[3], pl.maps[4], pl.maps[5], p));
         MUGD_CHECK_CUDA(launch_k(gemm_tc_reduce_kernel<BN, EPI>, dim3((unsigned)(p.gx * p.gy * TcReduceGeom<BN>::BPT)), dim3(TC_THREADS), 0, st, p));
@@ -316,23 +298,12 @@ static int tc_launch(const TcPlanned& pl, cudaStream_t st) {
     }
     if constexpr (BN == 128) {
         if (p.occ == 2) {
-            static bool configured2 = false;
-            if (!configured2) {
-                MUGD_CHECK_CUDA(cudaFuncSetAttribute(gemm_tc_kernel<BN, EPI, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TcSmem<BN, 2>::TOTAL));
-                MUGD_CHECK_CUDA(cudaFuncSetAttribute(gemm_tc_kernel<BN, EPI, 2>, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
-                configured2 = true;
-            }
             const int n_tiles = p.gx * p.gy;
             const int ctas = n_tiles < 2 * p.sm_count ? n_tiles : 2 * p.sm_count;
             MUGD_CHECK_CUDA(launch_k(gemm_tc_kernel<BN, EPI, 2>, dim3(ctas, 1, 1), dim3(TC_THREADS), TcSmem<BN, 2>::TOTAL, st, pl.maps[0], pl.maps[1],
                                      pl.maps[2], pl.maps[3], pl.maps[4], pl.maps[5], p));
             return MUGD_OK;
         }
-    }
-    static bool configured = false;
-    if (!configured) {
-        MUGD_CHECK_CUDA(cudaFuncSetAttribute(gemm_tc_kernel<BN, EPI>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TcSmem<BN>::TOTAL));
-        configured = true;
     }
     MUGD_CHECK_CUDA(launch_k(gemm_tc_kernel<BN, EPI>, dim3(p.gx, p.gy, 1), dim3(TC_THREADS), TcSmem<BN>::TOTAL, st, pl.maps[0], pl.maps[1],
                              pl.maps[2], pl.maps[3], pl.maps[4], pl.maps[5], p));
@@ -353,6 +324,24 @@ static int tc_launch_bn(const TcPlanned& pl, cudaStream_t st) {
     }
 }
 
+template <int BN, int OCC, int... EPI>
+static cudaError_t tc_configure(std::integer_sequence<int, EPI...>) {
+    cudaError_t e = cudaSuccess;
+    ((e = e != cudaSuccess ? e : cudaFuncSetAttribute(gemm_tc_kernel<BN, EPI, OCC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TcSmem<BN, OCC>::TOTAL)), ...);
+    if constexpr (OCC == 2) ((e = e != cudaSuccess ? e : cudaFuncSetAttribute(gemm_tc_kernel<BN, EPI, OCC>, cudaFuncAttributePreferredSharedMemoryCarveout, 100)), ...);
+    return e;
+}
+
+// every instantiation tc_launch can pick: 64 / 128 / 256 wide with each epilogue, and the 128-wide two-CTAs-per-SM variant
+int configure_gemm_tc_kernels(const DeviceInfo&) {
+    using Epis = std::make_integer_sequence<int, TC_E_COUNT>;
+    MUGD_CHECK_CUDA((tc_configure<64, 1>(Epis{})));
+    MUGD_CHECK_CUDA((tc_configure<128, 1>(Epis{})));
+    MUGD_CHECK_CUDA((tc_configure<256, 1>(Epis{})));
+    MUGD_CHECK_CUDA((tc_configure<128, 2>(Epis{})));
+    return MUGD_OK;
+}
+
 int launch_gemm_tc(const DeviceInfo& dev, const mugd_gemm& g, cudaStream_t st, int* launches) {
     TcPlanned pl;
     int rc = tc_plan(dev, g, &pl);
@@ -366,19 +355,6 @@ int launch_gemm_tc(const DeviceInfo& dev, const mugd_gemm& g, cudaStream_t st, i
 }
 
 }  // namespace mugd
-
-extern "C" int mugd_debug_set_tc_cost(float kstep128_us, float kstep256_us, float split_us, float two_cta_fixed_us) {
-    if (two_cta_fixed_us != 0.f) mugd::g_tc_cost[3] = two_cta_fixed_us;      // may be negative (a credit); 1e9 = never
-    if (kstep128_us > 0.f) mugd::g_tc_cost[0] = kstep128_us;
-    if (kstep256_us > 0.f) mugd::g_tc_cost[1] = kstep256_us;
-    if (split_us > 0.f) mugd::g_tc_cost[2] = split_us;
-    return MUGD_OK;
-}
-
-extern "C" int mugd_debug_set_tc_tile_n(int bn) {
-    mugd::g_tc_force_bn = (bn == 64 || bn == 128 || bn == 256 || bn == 130 /* 128 wide, two CTAs per SM */) ? bn : 0;
-    return MUGD_OK;
-}
 
 extern "C" int mugd_debug_set_tc_timing(long long* device_buf) {
 #ifdef MUGD_TC_TIMELINE

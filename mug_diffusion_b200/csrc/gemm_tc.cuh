@@ -424,8 +424,8 @@ struct TcBars {
 // (TcSmem<BN>::TILE_BYTES + barrier block), `tmem_base` = allocated tensor memory (>= TcSmem<BN>::TMEM_NEED columns), barriers
 // armed by the caller (TcBars::init) and visible to all threads.  All 256 threads call it; on return every TMA has landed, every
 // MMA has retired and been observed, and the tile (or its partial) is on its way to global memory.
-// PDL: stand-alone launches pass true -- the producer side executes griddepcontrol.wait before touching activations.
-template <int BN, bool PDL, int EPI, int OCC = 1>
+// The producer side executes griddepcontrol.wait (PDL) before touching activations.
+template <int BN, int EPI, int OCC = 1>
 __device__ __forceinline__ void gemm_tc_tile(const CUtensorMap* tmA, const CUtensorMap* tmA1, const CUtensorMap* tmA2, const CUtensorMap* tmB,
                                              const CUtensorMap* tmWhi, const CUtensorMap* tmWlo, const TcParams& p, int bx, int by, int bz,
                                              uint32_t base, uint32_t tmem_base, int it0 = 0, uint32_t acc_phase = 0) {
@@ -463,7 +463,7 @@ __device__ __forceinline__ void gemm_tc_tile(const CUtensorMap* tmA, const CUten
         if (p.hot.splits != 1) return;
         const int nn = n0 + ((int)threadIdx.x % (BN / 4)) * 4;
         if (g.step || (g.bias && nn < g.N)) {
-            if constexpr (PDL) pdl_wait();                       // the step counter is written by the previous kernels
+            pdl_wait();                                          // the step counter is written by the previous kernels
             if (g.step) epi_step = *g.step;
             if (g.bias && nn < g.N) epi_bias = ld_f4(g.bias + nn);
         }
@@ -494,7 +494,7 @@ __device__ __forceinline__ void gemm_tc_tile(const CUtensorMap* tmA, const CUten
                     tma_load_2d(b_hi(s), tmWhi, B.full(s), it * TC_BK, n0);
                     if (!h.single_pass) tma_load_2d(b_lo(s), tmWlo, B.full(s), it * TC_BK, n0);
                 }
-                if (PDL && i == 0) pdl_wait();      // activations written by the previous kernel are touched from here on
+                if (i == 0) pdl_wait();             // activations written by the previous kernel are touched from here on
                 if (it < h.it_main) {
                     const int t = it / h.kblocks;
                     const int kb = it - t * h.kblocks;
@@ -576,7 +576,7 @@ __device__ __forceinline__ void gemm_tc_tile(const CUtensorMap* tmA, const CUten
         // LayerNorm folded into this GEMM: fetch the moments of this thread's row now (written by earlier kernels), use them after the loop
         double ln_s = 0.0, ln_ss = 0.0;
         if constexpr (TcEpiTraits<EPI>::MODE == TC_EPI_LN) {
-            if constexpr (PDL) pdl_wait();
+            pdl_wait();
             const int rr = (warp & 3) * 32 + lane;
             if (rr < rows_valid && m_base + rr < g.M) {
                 const double2 mo = *reinterpret_cast<const double2*>(g.ln_stats + (int64_t)(m_base + rr) * 2);

@@ -175,7 +175,6 @@ constexpr int LN_MAXQ = 8;   // float4 per lane
 __global__ void __launch_bounds__(LN_WARPS * 32)
 layernorm_kernel(const float* __restrict__ x, int64_t ldx, float* __restrict__ y, int64_t ldy,
                  const float* __restrict__ gamma, const float* __restrict__ beta, int rows, int C, float eps) {
-    pdl_trigger();
     pdl_wait();
     const int row = blockIdx.x * LN_WARPS + (threadIdx.x >> 5);
     if (row >= rows) return;

@@ -22,7 +22,7 @@ struct PtrField { int kind; size_t off; };
 static const PtrField k_ptr_fields[] = {
     PF(MUGD_OP_GEMM, gemm.A), PF(MUGD_OP_GEMM, gemm.W), PF(MUGD_OP_GEMM, gemm.W_hi), PF(MUGD_OP_GEMM, gemm.W_lo), PF(MUGD_OP_GEMM, gemm.bias),
     PF(MUGD_OP_GEMM, gemm.rowvec), PF(MUGD_OP_GEMM, gemm.step), PF(MUGD_OP_GEMM, gemm.residual), PF(MUGD_OP_GEMM, gemm.C),
-    PF(MUGD_OP_GEMM, gemm.workspace), PF(MUGD_OP_GEMM, gemm.counters), PF(MUGD_OP_GEMM, gemm.A2), PF(MUGD_OP_GEMM, gemm.row_moments),
+    PF(MUGD_OP_GEMM, gemm.workspace), PF(MUGD_OP_GEMM, gemm.A2), PF(MUGD_OP_GEMM, gemm.row_moments),
     PF(MUGD_OP_GEMM, gemm.ln_stats), PF(MUGD_OP_GEMM, gemm.ln_colsum),
     PF(MUGD_OP_GROUPNORM, gn.x), PF(MUGD_OP_GROUPNORM, gn.y), PF(MUGD_OP_GROUPNORM, gn.gamma), PF(MUGD_OP_GROUPNORM, gn.beta),
     PF(MUGD_OP_LAYERNORM, ln.x), PF(MUGD_OP_LAYERNORM, ln.y), PF(MUGD_OP_LAYERNORM, ln.gamma), PF(MUGD_OP_LAYERNORM, ln.beta),

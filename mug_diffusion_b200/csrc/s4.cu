@@ -123,18 +123,19 @@ s4conv_kernel(const mugd_s4conv s, int nsplit, int Lpad) {
     }
 }
 
+// the byte count grows with L: allow what the device allows, the launcher checks each launch against it
+int configure_s4_kernels(const DeviceInfo& dev) {
+    MUGD_CHECK_CUDA(cudaFuncSetAttribute(s4conv_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, dev.max_smem_optin));
+    MUGD_CHECK_CUDA(cudaFuncSetAttribute(s4conv_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, dev.max_smem_optin));
+    return MUGD_OK;
+}
+
 int launch_s4conv(const DeviceInfo& dev, const mugd_s4conv& s, cudaStream_t st, int* launches) {
     MUGD_REQUIRE(s.B > 0 && s.L > 0 && s.H > 0 && s.H % S4_CH == 0, "s4conv: H=%d must be a positive multiple of %d", s.H, S4_CH);
     MUGD_REQUIRE(s.ldu >= s.H && s.ldy >= s.H, "s4conv: ld < H");
     const int Lpad = (s.L + 2 * S4_R - 1) / (2 * S4_R) * (2 * S4_R);
     const size_t smem = ((size_t)(S4_PAD + Lpad) + (size_t)(Lpad + 3 * S4_R)) * S4_PITCH * sizeof(float);
     MUGD_REQUIRE((int)smem <= dev.max_smem_optin, "s4conv: L=%d needs %zu B of shared memory (max %d)", s.L, smem, dev.max_smem_optin);
-    static bool configured = false;
-    if (!configured) {
-        MUGD_CHECK_CUDA(cudaFuncSetAttribute(s4conv_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, dev.max_smem_optin));
-        MUGD_CHECK_CUDA(cudaFuncSetAttribute(s4conv_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, dev.max_smem_optin));
-        configured = true;
-    }
     const int base = (s.H / S4_CH) * s.B;
     const int npairs = (Lpad / (2 * S4_R) + 1) / 2;
     int nsplit = 1;

@@ -90,15 +90,15 @@ class OpList:
              mode: int = L_.CONV_NONE, Lin: int = 0, Lout: int = 0, act: int = L_.ACT_NONE,
              gate: int = L_.GATE_NONE, residual: Optional[View] = None, rowvec: int = 0,
              rowvec_b_stride: int = 0, rowvec_step_stride: int = 0, step: int = 0, impl: int = L_.GEMM_AUTO,
-             W_hi: int = 0, W_lo: int = 0, split_k: int = 0, tap_shift: int = 0, dilation: int = 1, tag: int = 0,
-             A2: Optional[View] = None, ln: Optional[Tuple[int, int, float]] = None) -> int:
+             W_hi: int = 0, W_lo: int = 0, split_k: int = 0, tc_variant: int = L_.TC_AUTO, tap_shift: int = 0, dilation: int = 1,
+             tag: int = 0, A2: Optional[View] = None, ln: Optional[Tuple[int, int, float]] = None) -> int:
         g = L_.Gemm()
         M = out.rows
         g.A, g.lda = A.ptr, A.ld
         if not W_hi and W in self.tc_map:
             W_hi, W_lo = self.tc_map[W]
         g.W, g.W_hi, g.W_lo, g.bias = W, W_hi or None, W_lo or None, bias or None
-        g.split_k = split_k
+        g.split_k, g.tc_variant = split_k, tc_variant
         g.tap_shift = tap_shift
         g.tap_dilation = dilation
         g.rowvec, g.rowvec_b_stride, g.rowvec_step_stride = rowvec or None, rowvec_b_stride, rowvec_step_stride

@@ -19,7 +19,8 @@ CONV_NONE, CONV_SAME, CONV_DOWN, CONV_UP, CONV_TAPS = range(5)
 ACT_NONE, ACT_SILU, ACT_GELU = range(3)
 GATE_NONE, GATE_GEGLU, GATE_GLU = range(3)
 GEMM_AUTO, GEMM_SIMT, GEMM_TC = range(3)
-ABI_VERSION = 12
+TC_AUTO, TC_N64, TC_N128, TC_N256, TC_N128_2CTA = range(5)
+ABI_VERSION = 13
 
 _f = C.c_void_p  # device pointers travel as integers
 
@@ -31,9 +32,9 @@ class Gemm(C.Structure):
                 ("M", C.c_int32), ("N", C.c_int32), ("K", C.c_int32),
                 ("taps", C.c_int32), ("conv_mode", C.c_int32), ("Lin", C.c_int32), ("Lout", C.c_int32),
                 ("act", C.c_int32), ("gate", C.c_int32), ("impl", C.c_int32),
-                ("split_k", C.c_int32), ("n_counters", C.c_int32), ("tap_shift", C.c_int32), ("tap_dilation", C.c_int32),
-                ("workspace", _f), ("workspace_bytes", C.c_int64), ("counters", _f),
-                ("A2", _f), ("lda2", C.c_int64), ("K2", C.c_int32), ("reserved_", C.c_int32),
+                ("split_k", C.c_int32), ("tap_shift", C.c_int32), ("tap_dilation", C.c_int32),
+                ("workspace", _f), ("workspace_bytes", C.c_int64),
+                ("A2", _f), ("lda2", C.c_int64), ("K2", C.c_int32), ("tc_variant", C.c_int32),
                 ("row_moments", _f),
                 ("ln_stats", _f), ("ln_colsum", _f), ("ln_eps", C.c_float), ("reserved2_", C.c_int32)]
 
@@ -155,7 +156,6 @@ def load() -> C.CDLL:
     lib.mugd_gemm_tc_variant.argtypes = [C.POINTER(Gemm), C.c_int32, C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.POINTER(C.c_int32)]
     lib.mugd_gemm_tc_query.argtypes = [C.c_void_p, C.POINTER(Gemm), C.c_int32, C.POINTER(C.c_int32), C.POINTER(C.c_int32),
                                        C.POINTER(C.c_int64), C.POINTER(C.c_int32)]
-    lib.mugd_set_pdl.argtypes = [C.c_int]
     lib.mugd_debug_set_tc_timing.argtypes = [C.c_void_p]
     lib.mugd_fill_i32.argtypes = [C.c_void_p, C.c_int32, C.c_void_p]
     lib.mugd_abi_sizes.argtypes = [C.POINTER(C.c_int32), C.c_int32]
@@ -171,17 +171,6 @@ def load() -> C.CDLL:
     lib.mugd_plan_load.argtypes = [C.c_void_p, C.c_char_p, C.POINTER(Region), C.c_int32, C.POINTER(C.c_void_p)]
     lib.mugd_set_tc_single_pass_tf32.argtypes = [C.c_void_p, C.c_int]
     lib.mugd_set_attention_impl.argtypes = [C.c_void_p, C.c_int]
-    lib.mugd_debug_set_tc_tile_n.argtypes = [C.c_int]
-    lib.mugd_debug_set_tc_cost.argtypes = [C.c_float, C.c_float, C.c_float, C.c_float]
-    # measurement switches for tuning sweeps (tools/); none of them changes results
-    if os.environ.get("MUGD_TC_COST"):
-        lib.mugd_debug_set_tc_cost(*([float(v) for v in os.environ["MUGD_TC_COST"].split(",")] + [0.0] * 4)[:4])
-    if os.environ.get("MUGD_TC_TILE"):                       # experiments: force the tile variant (64 / 128 / 256 / 130 = 128 x two CTAs per SM)
-        lib.mugd_debug_set_tc_tile_n(int(os.environ["MUGD_TC_TILE"]))
-    if os.environ.get("MUGD_TC_BN"):
-        lib.mugd_debug_set_tc_tile_n(int(os.environ["MUGD_TC_BN"]))
-    if os.environ.get("MUGD_PDL") in ("0", "1"):
-        lib.mugd_set_pdl(int(os.environ["MUGD_PDL"]))
     _lib = lib
     return lib
 
@@ -199,6 +188,5 @@ EXPORTED_SYMBOLS = [
     "mugd_abi_version", "mugd_last_error", "mugd_create", "mugd_destroy", "mugd_device_info", "mugd_set_gemm_impl",
     "mugd_op_run", "mugd_plan_create", "mugd_plan_run", "mugd_plan_capture", "mugd_plan_replay",
     "mugd_plan_launch_count", "mugd_plan_destroy", "mugd_s4_kernel_gen", "mugd_fill_i32", "mugd_abi_sizes", "mugd_gemm_tc_query",
-    "mugd_set_pdl", "mugd_set_tc_single_pass_tf32", "mugd_set_attention_impl", "mugd_debug_set_tc_tile_n", "mugd_debug_set_tc_cost", "mugd_gemm_tc_variant",
-    "mugd_debug_set_attention_dump", "mugd_debug_set_tc_timing", "mugd_sample", "mugd_plan_save", "mugd_plan_load", "mugd_plan_regions", "mugd_plan_ops",
+    "mugd_set_tc_single_pass_tf32", "mugd_set_attention_impl", "mugd_gemm_tc_variant", "mugd_debug_set_tc_timing", "mugd_sample", "mugd_plan_save", "mugd_plan_load", "mugd_plan_regions", "mugd_plan_ops",
 ]

@@ -83,7 +83,6 @@ class MugEngine:
         # split-K scratch of the tensor-core GEMM: all ops run in stream order, so one buffer serves every plan
         # (bound: tiles*splits < 2*SMs tiles of 128x128 fp32)
         self.tc_ws = torch.zeros(8 * 1024 * 1024, device=self.device)          # 32 MB
-        self.tc_counters = torch.zeros(4096, dtype=torch.int32, device=self.device)
         # Compiled shapes are cached in small LRUs: webui derives z_length from each audio's duration (any multiple of
         # 32, webui.py:349-356), so an unbounded cache would grow by one ~1.5 GB arena + CUDA graph per new shape.
         self.sessions: "OrderedDict[tuple, Session]" = OrderedDict()
@@ -144,7 +143,6 @@ class MugEngine:
             if op.kind == L_.OP_GEMM:
                 g = op.u.gemm
                 g.workspace, g.workspace_bytes = self.tc_ws.data_ptr(), self.tc_ws.numel() * 4
-                g.counters, g.n_counters = self.tc_counters.data_ptr(), self.tc_counters.numel()
 
     def run_ops(self, ops: OpList):
         self.attach_workspace(ops)
@@ -402,7 +400,7 @@ class Session:
     def eval(self, graph: bool = True):
         if graph:
             if not self.plan.captured:
-                self.plan.run()               # warm-up (lazy module load, cudaFuncSetAttribute) outside capture
+                self.plan.run()               # warm-up (lazy module load) outside capture
                 self.plan.capture()
             self.plan.replay(1)
         else:
@@ -411,7 +409,7 @@ class Session:
     def run_steps(self, n: int, tail: OpList):
         """n DDIM steps from ONE C call (mugd_sample): n x {graph replay of the evaluation ; the tail ops (update, step advance)}"""
         if not self.plan.captured:
-            self.plan.run()                   # warm-up (lazy module load, cudaFuncSetAttribute) outside capture
+            self.plan.run()                   # warm-up (lazy module load) outside capture
             self.plan.capture()
         self.engine.attach_workspace(tail)
         arr = tail.array()
@@ -466,7 +464,7 @@ class DecoderSession:
         ops.transpose(_ptr(z), self.zin.ptr, 0, self.zin.ld, self.B, cfg.z_channels, self.Lz, True)
         eng.run_ops(ops)
         if not self.plan.captured:
-            self.plan.run()                   # warm-up (lazy module load, cudaFuncSetAttribute) outside capture
+            self.plan.run()                   # warm-up (lazy module load) outside capture
             self.plan.capture()
         self.plan.replay(1)
         out = torch.empty(self.B, cfg.x_channels, self.Lout, device=eng.device)

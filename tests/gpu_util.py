@@ -14,14 +14,12 @@ class OpRunner:
         L_.check(self.lib.mugd_create(0, C.byref(self.handle)), "mugd_create")
 
         self.ws = torch.zeros(16 * 1024 * 1024, device="cuda")
-        self.counters = torch.zeros(8192, dtype=torch.int32, device="cuda")
 
     def run(self, ops: OpList):
         for op in ops.ops:
             if op.kind == L_.OP_GEMM:
                 g = op.u.gemm
                 g.workspace, g.workspace_bytes = self.ws.data_ptr(), self.ws.numel() * 4
-                g.counters, g.n_counters = self.counters.data_ptr(), self.counters.numel()
         st = torch.cuda.current_stream().cuda_stream
         for op in ops.ops:
             L_.check(self.lib.mugd_op_run(self.handle, C.byref(op), st), f"op {op.kind}")

@@ -1,6 +1,9 @@
-"""Multi-GPU path on real devices (needs >= 2 GPUs; skipped otherwise): rank 0 packs, one NCCL broadcast of the blob, every rank
-samples its contiguous shard of the batch, logits are gathered on rank 0 -- and must equal the single-GPU run of the whole batch
-bit for bit (samples are independent; the per-rank plans have the same per-GPU batch as the chunks of the single-GPU reference)."""
+"""Multi-GPU paths on real devices (need >= 2 GPUs; skipped otherwise).
+* one process per GPU: rank 0 packs, one NCCL broadcast of the blob, every rank samples its contiguous shard of the batch, logits are
+  gathered on rank 0 -- and must equal the single-GPU run of the whole batch bit for bit (samples are independent; the per-rank plans
+  have the same per-GPU batch as the chunks of the single-GPU reference).
+* one process, one engine per GPU: libmugd state is per handle and kernel attributes are per device, so the engine on the second GPU
+  computes exactly what the first one does."""
 import os
 import socket
 
@@ -77,3 +80,38 @@ def test_two_rank_sharded_sampling_equals_single_gpu(tmp_path):
     single = torch.cat(chunks)
     assert gathered.shape == single.shape == (B, 16, 8 * L)
     assert torch.equal(gathered, single)
+
+
+def test_engines_on_two_devices_of_one_process_agree(golden_dir):
+    """The golden L=512 U-Net request four times over (Beff = 8) through session + eval on an engine on cuda:0 and one on cuda:1,
+    built from the same blob: every kernel with more than 48 KB of shared memory (tensor-core GEMM and attention, S4 conv) must launch
+    on the second device too, and both results must be bit-identical and match the reference's output."""
+    if torch.cuda.device_count() < 2:
+        pytest.skip("needs 2 GPUs")
+    import golden_cases as gc
+    from gpu_util import rel_err
+    from mug_diffusion_b200 import synth
+    from mug_diffusion_b200.config import ModelConfig
+    from mug_diffusion_b200.packer import pack_model
+    from mug_diffusion_b200.runtime import MugEngine
+
+    case, reps = gc.UNET_CASES["unet_L512_B2"], 4
+    L, Beff = case["L"], reps * case["B"]
+    cfg = ModelConfig()
+    blob = pack_model(synth.synthetic_state_dict(L), cfg.unet, cfg.decoder)
+    inp = synth.synthetic_inputs(case["B"], L)
+    eps = []
+    for d in (0, 1):
+        dev = torch.device(f"cuda:{d}")
+        with torch.cuda.device(dev):
+            eng = MugEngine(None, cfg, device=dev, blob=blob)
+            s = eng.session(Beff, L, per_sample_t=True)
+            s.set_timestep_table(case["t"] * reps)
+            s.set_context(torch.cat([inp["c"]] * reps).to(dev))
+            s.set_audio([torch.cat([w] * reps).to(dev) for w in inp["w"]])
+            s.load_x(torch.cat([inp["x_T"]] * reps).to(dev), dup=False)
+            s.eval()
+            eps.append(s.read_rows(s.eps, Beff, cfg.unet.out_channels, L).cpu())
+    assert torch.equal(eps[0], eps[1])
+    gold = gc.load_golden(os.path.join(golden_dir, "unet_L512_B2.npz"))["eps"]
+    assert rel_err(eps[1], torch.cat([gold] * reps)) < 1e-4

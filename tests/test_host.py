@@ -158,7 +158,7 @@ def test_synthetic_streams_are_stable():
 @pytest.mark.parametrize("Beff,Lz", [(2, 96), (8, 512), (64, 512), (16, 992)])
 def test_tensor_core_planner_invariants(packed, Beff, Lz):
     """tile / split-K planning of the tcgen05 GEMM (pure host code in libmugd, no GPU needed) over every GEMM of real plans:
-    what it takes it must be able to run with the engine's fixed 32 MB workspace and 4096 tile counters."""
+    what it takes it must be able to run with the engine's fixed 32 MB workspace."""
     import ctypes as C
     cfg, sd, blob = packed
     lib = L_.load()

@@ -1,5 +1,5 @@
 """Build an experiment variant of libmugd with extra -D defines into mug_diffusion_b200/libmugd_<name>.so
-usage: python tools/build_variant.py late -DMUGD_PDL_LATE_TRIGGER -DMUGD_PDL_SHORT_ENTRY ; then MUGD_LIB=<path> python bench.py ..."""
+usage: python tools/build_variant.py timeline -DMUGD_TC_TIMELINE ; then MUGD_LIB=<path> python tools/gemm_timeline.py"""
 import os
 import subprocess
 import sys

@@ -1,6 +1,6 @@
 """Where does one U-Net evaluation spend its device time?  Times every distinct op signature of the real launch plan
 in its own CUDA graph (REPS copies back to back, inputs warm in L2) and prints count x us per signature.
-usage (on the GPU box): python tools/profile_ops.py [--B 4] [--L 512] [--nocfg]"""
+usage (on the GPU box): python tools/profile_ops.py [--B 4] [--L 512] [--nocfg] [--tile 128x2]"""
 import argparse
 import collections
 import os
@@ -17,6 +17,7 @@ from mug_diffusion_b200.runtime import Plan  # noqa: E402
 from mug_diffusion_b200.sampler import MugDiffusionB200  # noqa: E402
 
 NAMES = {1: "gemm", 2: "groupnorm", 3: "layernorm", 4: "attention", 5: "s4conv", 7: "transpose", 8: "copy2d"}
+TILES = {"auto": L_.TC_AUTO, "64": L_.TC_N64, "128": L_.TC_N128, "256": L_.TC_N256, "128x2": L_.TC_N128_2CTA}
 
 
 def signature(op):
@@ -50,6 +51,8 @@ def main():
     ap.add_argument("--fuse", type=int, default=1, help="0: stand-alone LayerNorm kernels")
     ap.add_argument("--attn", type=int, default=1, help="0: exact-fp32 FFMA attention kernel instead of the tcgen05 one")
     ap.add_argument("--only", default="", help="only ops whose family name contains this")
+    ap.add_argument("--tile", choices=list(TILES), default="auto",
+                    help="force this tensor-core GEMM tile variant where the shape allows it (128x2: 128 wide, two CTAs per SM)")
     a = ap.parse_args()
     dev = torch.device("cuda:0")
     cfg = ModelConfig()
@@ -67,6 +70,8 @@ def main():
         if a.only and a.only not in sig[0]:
             continue
         sub = OpList()
+        if sig[0] == "gemm":
+            arr[idx[0]].u.gemm.tc_variant = TILES[a.tile]
         for _ in range(a.reps):
             sub.ops.append(arr[idx[0]])
         pl = Plan(eng, sub)
