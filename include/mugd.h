@@ -73,7 +73,8 @@ enum mugd_gate { MUGD_GATE_NONE = 0, MUGD_GATE_GEGLU = 1 /* a*gelu(g), attention
 enum mugd_gemm_impl { MUGD_GEMM_AUTO = 0, MUGD_GEMM_SIMT = 1 /* exact fp32 FMA */,
                       MUGD_GEMM_TC = 2 /* tcgen05 3xTF32 split, fp32 accumulate in TMEM */ };
 /* tile variant of the tensor-core GEMM (mugd_gemm.tc_variant): AUTO = the planner's cost model; the others force a variant where
- * the shape allows it (a tile wider than N falls back to the 128- or 64-wide tile) */
+ * the shape allows it (a tile wider than N falls back to the 128- or 64-wide tile; N128_2CTA together with split_k > 1 falls back to
+ * the 128-wide one-CTA-per-SM tile with that split) */
 enum mugd_tc_variant { MUGD_TC_AUTO = 0, MUGD_TC_N64 = 1, MUGD_TC_N128 = 2, MUGD_TC_N256 = 3,
                        MUGD_TC_N128_2CTA = 4 /* 128 wide, two CTAs per SM walking a tile list */ };
 

@@ -160,8 +160,10 @@ TcGeometry tc_geometry(const mugd_gemm& g, int sm_count, int forced_split) {
     int splits = 1;
     float best = 1e30f;
     static const int cands[4] = {64, 128, 256, 130 /* 128 wide, two CTAs per SM */};
-    // a forced variant (mugd_gemm.tc_variant) in the same codes; 0 = cost model
-    const int force = (g.tc_variant >= MUGD_TC_N64 && g.tc_variant <= MUGD_TC_N128_2CTA) ? cands[g.tc_variant - MUGD_TC_N64] : 0;
+    // a forced variant (mugd_gemm.tc_variant) in the same codes; 0 = cost model.  The two-CTA variant has no split-K form: with a
+    // forced split it falls back to the 128-wide one-CTA-per-SM tile, which honours the split.
+    int force = (g.tc_variant >= MUGD_TC_N64 && g.tc_variant <= MUGD_TC_N128_2CTA) ? cands[g.tc_variant - MUGD_TC_N64] : 0;
+    if (force == 130 && forced_split > 1) force = 128;
     for (int cand = 0; cand < 4; ++cand) {
         const int code = cands[cand];
         const int bn = code == 130 ? 128 : code;

@@ -166,8 +166,8 @@ def test_upsample_as_two_parity_gemms(R, impl, B, L, C):
 
 @pytest.mark.parametrize("kind", ["linear", "conv3"])
 def test_tc_oversubscribed_grid(R, kind):
-    """grids of several waves (more tiles than the 148 SMs, 256-wide tiles with the decoupled weight ring where N allows):
-    same numbers as the fp64 reference"""
+    """grids with more tiles than the 148 SMs, as the cost model plans them (both cases run the 128-wide two-CTA variant; the
+    256-wide tiles are pinned in test_gpu_gemm_matrix.py): same numbers as the fp64 reference"""
     if kind == "linear":
         M, K, N = 296 * 128, 128, 256
         x, w, b = g("mcx", (M, K)), g("mcw", (N, K)) / math.sqrt(K), 0.1 * g("mcb", (N,))
